@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- grasps/sec of the PointNet grasp-quality hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config train|infer|tower]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config train|infer|tower] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Default (`--config train`): one "step" = one pass of the hot path over one batch of synthetic grasp clouds: forward
@@ -12,6 +12,10 @@ its own batch.  Other BASELINE configs: `--classes 3` (config 3), `--batch 128 -
 shape: 1024 clouds x 1024 points through pgpd_tower_forward).
 
 Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for how each field is produced.
+
+`--dump-outputs DIR` writes what the last timed step returned to its caller as DIR/<name>.npy (float32 / float64): the
+log-probs (infer), the pooled features (tower), or the loss plus every parameter and BatchNorm buffer after the update
+(train).  The inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import ctypes
@@ -31,6 +35,22 @@ if ROOT not in sys.path:
 
 UNIT = "grasps/s"
 CPU_SAMPLE_B = 128        # clouds per step of the CPU arms (a bounded sample of the 512-cloud workload)
+DUMP_BUDGET = 64 << 20    # bytes of --dump-outputs in all
+
+
+def dump_outputs(out_dir, arrays):
+    """Write {name: host tensor} as out_dir/<name>.npy.  An array larger than its even share of DUMP_BUDGET is cut to a
+    fixed, seeded sample of its rows (sorted, so the order matches the full output), so the dump stays comparable."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BUDGET // max(1, len(arrays))
+    for name, t in arrays.items():
+        a = t.numpy()
+        a = a.astype(np.float32 if a.dtype == np.float32 else np.float64).reshape(a.shape or (1,))
+        if a.nbytes > share:
+            rows = max(1, share // max(1, a[0].nbytes))
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], size=rows, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def load_peaks():
@@ -223,7 +243,13 @@ def main():
     ap.add_argument("--simt", action="store_true", help="force the fp32 CUDA-core kernels")
     ap.add_argument("--no-graph", action="store_true", help="launch every step eagerly instead of replaying a CUDA graph")
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the CPU / eager-GPU baseline legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/<name>.npy (at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.batch is None:
         args.batch = {"train": 512, "infer": 4096, "tower": 1024}[args.config]
     if args.points is None:
@@ -241,12 +267,12 @@ def main():
         if rank != 0:
             return 0
         torch.set_num_threads(host_threads())
-        steps, warm = max(1, args.steps), max(1, args.warmup)
+        steps, warm = args.steps, max(1, args.warmup)
         if args.config == "train":
-            r = port_train_arm("cpu", CPU_SAMPLE_B, N, k, steps, warm, max_seconds=170.0)
+            r = port_train_arm("cpu", CPU_SAMPLE_B, N, k, steps, warm)
             what = "fwd+nll+bwd+Adam"
         else:
-            r = port_infer_arm("cpu", CPU_SAMPLE_B, N, k, min(steps, 10), min(warm, 2))
+            r = port_infer_arm("cpu", CPU_SAMPLE_B, N, k, steps, min(warm, 2))
             what = "eval forward"
         line = {"impl": "reference", "metric": metric, "value": r["value"], "unit": UNIT, "n_gpus": args.gpus,
                 "steps": r["steps_done"], "warmup": warm, "ms_per_step": r["ms_per_step"], "higher_is_better": True,
@@ -469,10 +495,19 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for i in range(args.steps):
-        dev_step(i)
+        last = dev_step(i)
     e1.record()
     barrier()
     ms_total = e0.elapsed_time(e1)
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        # snapshot before the end-to-end region below runs further steps on the same model and buffers
+        if args.config == "train":
+            dumped = {"loss": last.detach().float().cpu()}
+            dumped.update({"param." + n: p.detach().cpu().clone() for n, p in model.named_parameters()})
+            dumped.update({"buffer." + n: b.detach().cpu().clone() for n, b in model.named_buffers()})
+        else:
+            dumped = {"logp" if args.config == "infer" else "pooled": last.detach().cpu().clone()}
     launches = int(lib.pgpd_launch_count() - n0)
     nl, tot = ctypes.c_int(0), ctypes.c_float(0.0)
     lib.pgpd_profile_read(ctypes.byref(nl), ctypes.byref(tot))      # graph mode: the event nodes of the LAST replayed step
@@ -580,6 +615,8 @@ def main():
                     line["gpu_eager_baseline"] = {"fp32": {"value": r2["value"], "unit": UNIT, "ms_per_step": r2["ms_per_step"]},
                                                   "what": "eager PyTorch (oracle torch port) eval forward on the same GPU, fp32"}
         print(json.dumps(line), flush=True)
+        if dumped is not None:
+            dump_outputs(args.dump_outputs, dumped)
     if world > 1:
         # the line is out; never let communicator teardown hang the job
         threading.Timer(30.0, lambda: os._exit(0)).start()

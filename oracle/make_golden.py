@@ -3,18 +3,17 @@
 
 TEST INFRASTRUCTURE ONLY (see oracle/__init__.py).
 
-Run in the build container only (needs /root/reference):
-    python oracle/make_golden.py
-It imports /root/reference/PointNetGPD/model/pointnet.py (PointNetCls, :177-194),
+Run where a checkout of the reference project is available:
+    python oracle/make_golden.py /path/to/reference-checkout
+(the directory that holds PointNetGPD/ and data/).  It imports PointNetGPD/model/pointnet.py (PointNetCls, :177-194),
 loads deterministic weights from oracle.weights, runs forward / nll_loss /
 backward exactly as main_1v.py:72-75 does, and stores inputs-by-recipe plus
 outputs.  Nothing is copied from the reference: the fixtures hold numbers only.
 
-Also extracts the tensors of the shipped checkpoint
-(/root/reference/data/pointnetgpd_3class.model, a pickled
-DataParallel(PointNetCls(num_points=500, k=3)), SURVEY.md Appendix B) into
-tests/golden/shipped_3class_state.npz so that the real-weights known-answer test
-can run on the GPU box, where /root/reference does not exist.
+Also reduces the shipped checkpoint (data/pointnetgpd_3class.model, a pickled
+DataParallel(PointNetCls(num_points=500, k=3)), SURVEY.md Appendix B) to a fixture
+under 1 MB (run_shipped) and records the reference's outputs on it, so that the
+real-statistics known-answer tests run without the reference.
 """
 import os
 import sys
@@ -29,7 +28,8 @@ ROOT = os.path.dirname(HERE)
 sys.path.insert(0, ROOT)
 from oracle import weights as W  # noqa: E402
 
-REF = "/root/reference/PointNetGPD"
+REF_ROOT = None        # the reference checkout, set by main()
+REF = None             # REF_ROOT/PointNetGPD
 GOLD = os.path.join(ROOT, "tests", "golden")
 
 # (name, B, N, k, weight style, cloud kind, seed)
@@ -121,20 +121,105 @@ def run_case(PointNetCls, name, B, N, k, style, kind, seed):
     print("wrote", name, "loss f32 %.7f f64 %.12f" % (out["train_loss_f32"], out["train_loss_f64"]))
 
 
+# The six largest matrices of the shipped checkpoint (1.57 M of its 1.61 M values) do not fit a 1 MB fixture.  The fixture
+# keeps every other tensor exactly (BatchNorm statistics with negative gammas and extreme running variances, biases, the
+# first two convolutions, the last FC layers) and replaces these by seeded draws with each output row's mean and std.
+SHIPPED_BIG = ("feat.stn.conv3.weight", "feat.stn.fc1.weight", "feat.stn.fc2.weight", "feat.conv3.weight", "fc1.weight",
+               "fc2.weight")
+
+
+def load_shipped_state(path):
+    """The 74-entry state dict of the reduced shipped checkpoint stored at `path` (tests/golden/shipped_3class_state.npz)."""
+    z = np.load(path)
+    sd = {k: z[k] for k in z.files if "/" not in k}
+    for i, k in enumerate(SHIPPED_BIG):
+        mean, std = z["rowmean/" + k], z["rowstd/" + k]
+        shape = tuple(int(n) for n in z["shape/" + k])
+        rows = mean[:, None] + std[:, None] * W.normal(9000 + i, (shape[0], int(np.prod(shape[1:]))))
+        sd[k] = rows.reshape(shape).astype(np.float32)
+    return sd
+
+
+def write_shipped_pickle(path, head, storage_keys, sd):
+    """Reassemble the legacy torch.save file of the shipped checkpoint from its object pickle (`head`: everything up to the
+    table of storages) and the tensors of `sd`, each storage written as torch's legacy format does: int64 numel, raw data."""
+    with open(path, "wb") as f:
+        f.write(head.tobytes())
+        for key in storage_keys:
+            v = np.ascontiguousarray(sd[str(key)])
+            f.write(np.int64(v.size).tobytes())
+            f.write(v.tobytes())
+
+
+def _shipped_pickle_head(path, sd):
+    """The checkpoint's legacy-format header and object pickle, with the class source texts and file paths torch.save
+    embedded in it blanked (torch.load only compares them to warn about changed sources), and the state key of every
+    storage in file order."""
+    import pickle
+    import pickletools
+    with open(path, "rb") as f:
+        for _ in range(3):                      # magic number, protocol version, sys_info
+            pickle.load(f)
+        obj_start = f.tell()
+        blank = set()
+
+        class Probe(pickle.Unpickler):
+            def find_class(self, mod, name):
+                return super().find_class(mod, name) if mod == "collections" else type(name, (), {"__init__": lambda s, *a, **k: None, "__setstate__": lambda s, st: None})
+
+            def persistent_load(self, pid):
+                if pid[0] == "module":
+                    blank.update(x for x in pid[2:] if x)
+                    return pid[1]
+                return None
+        Probe(f).load()
+        obj_end = f.tell()
+        keys = pickle.load(f)
+        data_start = f.tell()
+        f.seek(0)
+        raw = f.read()
+    obj = bytearray(raw[obj_start:obj_end])
+    for op, arg, pos in reversed(list(pickletools.genops(bytes(obj)))):
+        if op.name == "BINUNICODE" and arg in blank:
+            obj[pos:pos + 5 + len(arg.encode("utf-8"))] = b"X\x00\x00\x00\x00"
+    head = raw[:obj_start] + bytes(obj) + raw[obj_end:data_start]
+    # storage -> state key, by content (tensors with equal contents are interchangeable)
+    order, off = [], data_start
+    for _key in keys:
+        n = int(np.frombuffer(raw[off:off + 8], np.int64)[0])
+        off += 8
+        for name, v in sd.items():
+            if v.size == n and raw[off:off + v.nbytes] == np.ascontiguousarray(v).tobytes():
+                order.append(name)
+                off += v.nbytes
+                break
+        else:
+            raise RuntimeError("storage %s matches no state tensor" % _key)
+    assert off == len(raw)
+    return np.frombuffer(head, np.uint8), np.array(order)
+
+
 def run_shipped(PointNetCls):
-    path = "/root/reference/data/pointnetgpd_3class.model"
+    path = os.path.join(REF_ROOT, "data", "pointnetgpd_3class.model")
     model = torch.load(path, map_location="cpu", weights_only=False)   # main_test.py:42
     if isinstance(model, torch.nn.DataParallel):                         # main_test.py:55-56
         model = model.module
-    sd = {k: v.numpy() for k, v in model.state_dict().items()}
-    np.savez_compressed(os.path.join(GOLD, "shipped_3class_state.npz"), **sd)
-    # modern torch needs these attributes that 0.4-era pickles lack
-    fresh = PointNetCls(num_points=500, input_chann=3, k=3)
-    fresh.load_state_dict(model.state_dict())
+    full = {k: v.numpy() for k, v in model.state_dict().items()}
+    fx = {k: v for k, v in full.items() if k not in SHIPPED_BIG}
+    for k in SHIPPED_BIG:
+        rows = full[k].astype(np.float64).reshape(full[k].shape[0], -1)
+        fx["rowmean/" + k], fx["rowstd/" + k] = rows.mean(1).astype(np.float32), rows.std(1).astype(np.float32)
+        fx["shape/" + k] = np.array(full[k].shape, np.int64)
+    gold_state = os.path.join(GOLD, "shipped_3class_state.npz")
+    np.savez_compressed(gold_state, **fx)
+    sd_np = load_shipped_state(gold_state)
+    head, order = _shipped_pickle_head(path, full)
+    np.savez_compressed(os.path.join(GOLD, "shipped_3class_pickle.npz"), head=head, storage_keys=order)
+    sd = {k: torch.tensor(v) for k, v in sd_np.items()}
     out = {}
     for dtype, tag in ((torch.float32, "f32"), (torch.float64, "f64")):
-        m = PointNetCls(num_points=500, input_chann=3, k=3)
-        m.load_state_dict(model.state_dict())
+        m = PointNetCls(num_points=500, input_chann=3, k=3)               # modern torch needs attributes 0.4-era pickles lack
+        m.load_state_dict(sd)
         m = m.to(dtype).eval()
         for kind, seed in (("box", 123), ("dup", 124)):
             x = W.make_clouds(seed, 8, 500, kind)
@@ -224,7 +309,51 @@ def run_dual(only=False):
     print("wrote dual_b6_n72_k2; eval logp[0] =", out["eval_logp_f32"][0])
 
 
+def run_dual_pin():
+    """The reference DualPointNetCls on the inputs of tests/test_dual.py::test_dual_port_matches_reference: its state-dict
+    keys, eval and train-mode outputs in fp32, and the BatchNorm buffers after the train-mode forward."""
+    from model.pointnet import DualPointNetCls
+    st = W.make_state(3, k=3, style="wild", dual=True)
+    m = DualPointNetCls(40, 6, 3)
+    out = {"state_keys": np.array(list(m.state_dict().keys()))}
+    load_state(m, st)
+    x = torch.tensor(np.concatenate([W.make_clouds(1, 5, 40, "box"), W.make_clouds(1 + 77, 5, 40, "box")], axis=1))
+    for training, tag in ((False, "eval"), (True, "train")):
+        m.train(training)
+        logp, trans = m(x)
+        out[f"{tag}_logp"], out[f"{tag}_trans"] = logp.detach().numpy(), trans.detach().numpy()
+    for name, b in m.named_buffers():
+        out["buf/" + name] = b.numpy()
+    np.savez_compressed(os.path.join(GOLD, "dual_pin_b5_n40_k3.npz"), **out)
+    print("wrote dual_pin_b5_n40_k3")
+
+
+def run_gpd_pin():
+    """The reference GPDClassifier (PointNetGPD/model/gpd.py) in eval mode on the inputs of
+    tests/test_gpd.py::test_gpd_port_matches_reference, and its state-dict keys."""
+    import importlib.util
+    from oracle import gpd_torch_port as G
+    spec = importlib.util.spec_from_file_location("ref_gpd", os.path.join(REF, "model", "gpd.py"))
+    mod = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(mod)
+    out = {"state_keys": np.array(list(mod.GPDClassifier(3).state_dict().keys()))}
+    for Cc in (3, 12):
+        m = mod.GPDClassifier(Cc)
+        m.load_state_dict(G.make_gpd_state(5, Cc))
+        m.eval()
+        x = torch.tensor(W.normal(6, (3, Cc, 60, 60)).astype(np.float32))
+        with torch.no_grad():
+            out[f"logp_c{Cc}"] = m(x).numpy()
+    np.savez_compressed(os.path.join(GOLD, "gpd_pin.npz"), **out)
+    print("wrote gpd_pin")
+
+
 def main():
+    global REF_ROOT, REF
+    if len(sys.argv) < 2 or not os.path.isdir(os.path.join(sys.argv[1], "PointNetGPD")):
+        raise SystemExit("usage: python oracle/make_golden.py REFERENCE_CHECKOUT [--dual-only]")
+    REF_ROOT = os.path.abspath(sys.argv[1])
+    REF = os.path.join(REF_ROOT, "PointNetGPD")
     os.makedirs(GOLD, exist_ok=True)
     torch.set_num_threads(8)
     PointNetCls = _import_reference()
@@ -235,6 +364,8 @@ def main():
         run_case(PointNetCls, *case)
     run_shipped(PointNetCls)
     run_collect_pc()
+    run_dual_pin()
+    run_gpd_pin()
 
 
 if __name__ == "__main__":

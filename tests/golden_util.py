@@ -5,7 +5,7 @@ import os
 import numpy as np
 
 from oracle import weights as W
-from oracle.make_golden import sub_idx, CASES
+from oracle.make_golden import sub_idx, CASES, load_shipped_state
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 CASE_NAMES = [c[0] for c in CASES]
@@ -22,6 +22,11 @@ def load_case(name):
     wl = W.normal(seed + 3000, (B, k))
     wt = W.normal(seed + 4000, (B, 3, 3))
     return dict(g=g, B=B, N=N, k=k, seed=seed, state=state, x=x, y=y, wl=wl, wt=wt)
+
+
+def shipped_state():
+    """The 74-entry state dict of the shipped 3-class checkpoint, as reduced in tests/golden (oracle/make_golden.py)."""
+    return load_shipped_state(os.path.join(GOLDEN, "shipped_3class_state.npz"))
 
 
 def param_names(state):

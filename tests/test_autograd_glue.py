@@ -10,7 +10,7 @@ import pytest
 import torch
 
 import emu_util as E
-from golden_util import load_case, is_zero_grad_param
+from golden_util import load_case, is_zero_grad_param, shipped_state
 from oracle import pointnet_torch_port as PT
 from pointnetgpd_b200 import _abi as A
 from pointnetgpd_b200 import functional as Fn
@@ -160,13 +160,18 @@ def test_state_dict_keys_and_pickle_roundtrip():
     assert m.device_ids == [0]
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/data/pointnetgpd_3class.model"), reason="reference not mounted")
-def test_shipped_checkpoint_unpickles_into_our_classes(golden_dir):
+def test_shipped_checkpoint_unpickles_into_our_classes(golden_dir, tmp_path):
     """The 2018 whole-module pickle references `model.pointnet.{PointNetCls,PointNetfeat,STN3d}` (SURVEY App. B);
-    with install_as_model() those resolve to this package's classes, without running __init__."""
+    with install_as_model() those resolve to this package's classes, without running __init__.  The file is rebuilt from
+    the checkpoint's own object pickle and the tensors of the reduced fixture (oracle/make_golden.py)."""
     import sys
     import types
     import pointnetgpd_b200
+    from oracle.make_golden import write_shipped_pickle
+    ref = shipped_state()
+    fx = np.load(os.path.join(golden_dir, "shipped_3class_pickle.npz"))
+    path = str(tmp_path / "pointnetgpd_3class.model")
+    write_shipped_pickle(path, fx["head"], fx["storage_keys"], ref)
     saved = {k: sys.modules.get(k) for k in ("model", "model.pointnet", "model.gpd", "torch.nn.backends.thnn")}
     try:
         pointnetgpd_b200.install_as_model(force=True)
@@ -176,11 +181,10 @@ def test_shipped_checkpoint_unpickles_into_our_classes(golden_dir):
         import warnings
         with warnings.catch_warnings():
             warnings.simplefilter("ignore")
-            obj = torch.load("/root/reference/data/pointnetgpd_3class.model", map_location="cpu", weights_only=False)
+            obj = torch.load(path, map_location="cpu", weights_only=False)
         mod = obj.module if isinstance(obj, torch.nn.DataParallel) else obj
         assert type(mod) is PointNetCls and type(mod.feat.stn) is STN3d
         assert mod.num_points == 500 and mod.fc3.out_features == 3
-        ref = np.load(os.path.join(golden_dir, "shipped_3class_state.npz"))
         for k, v in mod.state_dict().items():
             assert np.array_equal(v.numpy(), ref[k]), k
         params, bufs = Fn.gather_tensors(mod, A.PGPD_CLS)

@@ -1,14 +1,8 @@
-"""Drop-in tests of the host-side mirror: dataset classes against the reference's collect_pc goldens, the synthetic
-dataset tree, and the launcher running the UNMODIFIED reference script (only where /root/reference is mounted)."""
+"""Drop-in tests of the host-side mirror: dataset classes against the reference's collect_pc goldens and the synthetic
+dataset tree."""
 import os
-import subprocess
-import sys
 
 import numpy as np
-import pytest
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_SCRIPT = "/root/reference/PointNetGPD/main_1v.py"
 
 
 def test_dataset_crop_matches_reference_golden(golden_dir):
@@ -43,15 +37,3 @@ def test_synthetic_tree_and_dataset_contract(tmp_path, monkeypatch):
     it = mc[3]
     assert it is not None and it[0].shape == (3, 1000) and it[1] in (0, 1, 2)
 
-
-@pytest.mark.skipif(not os.path.exists(REF_SCRIPT), reason="reference not mounted")
-def test_launcher_runs_unmodified_reference_script(tmp_path):
-    """main_1v.py, byte-identical, imported through the launcher: tensorboardX shim, `model.*` aliases, dataset
-    construction over a synthetic tree, PointNetCls construction.  `--epoch 0` makes its epoch loop empty, so the
-    script exits before the (GPU-only) forward pass -- the training step itself is covered by the GPU tests."""
-    env = dict(os.environ, PYTHONPATH=ROOT)
-    cmd = [sys.executable, "-m", "pointnetgpd_b200.launcher", "--synthetic-data", str(tmp_path / "tree"), REF_SCRIPT,
-           "--mode", "train", "--epoch", "0", "--batch-size", "16", "--tag", "dropin"]
-    res = subprocess.run(cmd, cwd=str(tmp_path), env=env, capture_output=True, text=True, timeout=300)
-    assert res.returncode == 0, res.stderr[-2000:]
-    assert os.path.isdir(tmp_path / "assets" / "learned_models")

@@ -8,7 +8,7 @@ import numpy as np
 import pytest
 import torch
 
-from golden_util import CASE_NAMES, load_case, grad_errors, is_zero_grad_param
+from golden_util import CASE_NAMES, load_case, grad_errors, is_zero_grad_param, shipped_state
 from oracle import pointnet_torch_port as PT
 from oracle import weights as W
 from pointnetgpd_b200 import _abi as A
@@ -79,8 +79,9 @@ def test_train_step_golden(name):
 
 
 def test_shipped_checkpoint_known_answer(golden_dir):
-    """Real trained weights (negative BN gammas, extreme running stats; SURVEY App. B): N=500, k=3."""
-    st = dict(np.load(os.path.join(golden_dir, "shipped_3class_state.npz")))
+    """The shipped checkpoint's trained BatchNorm layers (negative gammas, extreme running stats; SURVEY App. B), its largest
+    matrices resampled to fit the fixture (oracle/make_golden.py): N=500, k=3."""
+    st = shipped_state()
     out = np.load(os.path.join(golden_dir, "shipped_3class_outputs.npz"))
     m = _model(st, 500, 3, train=False)
     for kind, seed in (("box", 123), ("dup", 124)):

@@ -5,6 +5,7 @@ import numpy as np
 import pytest
 import torch
 
+from golden_util import shipped_state
 from oracle import grasp_crop_np as OC
 from oracle import pointnet_torch_port as PT
 from oracle import weights as W
@@ -61,7 +62,7 @@ def test_resample_gpu_properties():
 def test_score_candidates_matches_oracle(golden_dir):
     """deployment path (kinect2grasp.py:454-491) with the shipped 3-class checkpoint: batched GPU scoring vs the
     oracle evaluated on the same resampled points."""
-    st = dict(np.load(os.path.join(golden_dir, "shipped_3class_state.npz")))
+    st = shipped_state()
     m = PointNetCls(num_points=500, k=3)
     m.load_state_dict({k: torch.tensor(v) for k, v in st.items()})
     m = m.cuda().eval()

@@ -6,7 +6,7 @@ import torch
 
 from oracle import pointnet_np as PN
 from oracle import pointnet_torch_port as PT
-from golden_util import (CASE_NAMES, SMALL_CASES, load_case, param_names, grad_errors,
+from golden_util import (CASE_NAMES, SMALL_CASES, load_case, param_names, grad_errors, shipped_state,
                          is_zero_grad_param)
 
 
@@ -79,7 +79,7 @@ def test_numpy_fp64_general_output_grads(name):
 def test_shipped_checkpoint_known_answer(golden_dir):
     import os
     from oracle import weights as W
-    st = dict(np.load(os.path.join(golden_dir, "shipped_3class_state.npz")))
+    st = shipped_state()
     out = np.load(os.path.join(golden_dir, "shipped_3class_outputs.npz"))
     assert len(st) == 74
     sd = PT.to_torch_state(st, torch.float32)
