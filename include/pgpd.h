@@ -234,6 +234,23 @@ int pgpd_crop_box(const float* pc, int P, const double* frames, int G, const int
 int pgpd_resample(const float* pts, const int* offsets, int C, int N, int repeat, unsigned long long seed,
                   float* out_x, int* out_idx, void* stream);
 
+/* GPD image projection (BaseGraspDataset.project_pc / cal_projection, PointNetGPD/model/dataset.py:78-198) of one cloud
+ * for G grasps, after pgpd_crop_box:
+ *   pc, frames       : as for pgpd_crop_box
+ *   offsets, idx     : [G+1] segment bounds and [offsets[G]] ascending cloud indices of the in-box points (pgpd_crop_box)
+ *   chann            : 3 (normals of the [x,y,z] image) or 12 ([occupancy, normal] of the orders [0,1,2], [1,2,0], [0,2,1])
+ *   out              : [G][chann][60][60] fp32, the layout pgpd_gpd_forward reads (out[c][y][x] = the reference's
+ *                      image[x][y][c]); all zeros for a grasp with fewer than 50 in-box points
+ *   valid            : [G] bytes, 1 where the box holds >= 50 points (the reference's item is None otherwise)
+ * Normals: up to 30 nearest cloud points within distance 0.1 (itself included), covariance in the grasp frame (fp64),
+ * eigenvector of the smallest eigenvalue from the closed-form symmetric 3x3 solver; fewer than 3 neighbours or a zero
+ * covariance give (0,0,1).  Deterministic: the same inputs give bit-identical outputs.
+ * The workspace (256-byte aligned) comes from pgpd_gpd_project_workspace_bytes(P, G, offsets[G], chann); a grasp whose
+ * points lie beyond what the given workspace holds is written as NaN with valid = 0. */
+size_t pgpd_gpd_project_workspace_bytes(int P, int G, int total_in_box, int chann);
+int pgpd_gpd_project(const float* pc, int P, const double* frames, int G, const int* offsets, const int* idx, int chann,
+                     float* out, unsigned char* valid, void* workspace, size_t workspace_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -85,7 +85,7 @@ class DualGrad(C.Structure):
 EXPORTS = ("pgpd_dual_workspace_bytes", "pgpd_dual_forward", "pgpd_dual_backward", "pgpd_gpd_workspace_bytes", "pgpd_gpd_forward", "pgpd_gpd_backward", "pgpd_version", "pgpd_last_error", "pgpd_has_tensor_core_path", "pgpd_launch_count",
            "pgpd_profile_enable", "pgpd_profile_read", "pgpd_workspace_bytes",
            "pgpd_forward", "pgpd_backward", "pgpd_tower_workspace_bytes", "pgpd_tower_forward",
-           "pgpd_tower_backward", "pgpd_crop_box", "pgpd_resample")
+           "pgpd_tower_backward", "pgpd_crop_box", "pgpd_resample", "pgpd_gpd_project_workspace_bytes", "pgpd_gpd_project")
 
 
 def bind(lib):
@@ -134,6 +134,10 @@ def bind(lib):
     lib.pgpd_crop_box.argtypes = [_fp, C.c_int, _fp, C.c_int, _fp, _fp, _fp, _fp, _fp]
     lib.pgpd_resample.restype = C.c_int
     lib.pgpd_resample.argtypes = [_fp, _fp, C.c_int, C.c_int, C.c_int, C.c_ulonglong, _fp, _fp, _fp]
+    lib.pgpd_gpd_project_workspace_bytes.restype = C.c_size_t
+    lib.pgpd_gpd_project_workspace_bytes.argtypes = [C.c_int] * 4
+    lib.pgpd_gpd_project.restype = C.c_int
+    lib.pgpd_gpd_project.argtypes = [_fp, C.c_int, _fp, C.c_int, _fp, _fp, C.c_int, _fp, _fp, _fp, C.c_size_t, _fp]
     return lib
 
 

@@ -5,6 +5,7 @@
 #include "tower.cuh"
 #include "head.cuh"
 #include "prep.cuh"
+#include "project.cuh"
 #include "gpd.cuh"
 #include "dual.cuh"
 
@@ -421,6 +422,27 @@ int pgpd_resample(const float* pts, const int* offsets, int C, int N, int repeat
     if (!pts || !offsets || !out_x || C < 1 || N < 1 || repeat < 1) return fail(PGPD_E_ARG, "bad argument");
     launch(k_resample, dim3(C, repeat), dim3(256), 0, (cudaStream_t)stream, pts, offsets, N, seed, out_x, out_idx);
     return check_cuda("pgpd_resample");
+}
+
+size_t pgpd_gpd_project_workspace_bytes(int P, int G, int total_in_box, int chann) {
+    if (P < 0 || G < 1 || total_in_box < 0 || (chann != 3 && chann != 12)) return 0;
+    proj::ProjWs w;
+    proj::plan_project(nullptr, P, total_in_box, chann, w);
+    return w.bytes;
+}
+
+int pgpd_gpd_project(const float* pc, int P, const double* frames, int G, const int* offsets, const int* idx, int chann,
+                     float* out, unsigned char* valid, void* workspace, size_t workspace_bytes, void* stream) {
+    if (!pc || !frames || !offsets || !out || !valid || P < 0 || G < 1) return fail(PGPD_E_ARG, "bad argument");
+    if (chann != 3 && chann != 12) return fail(PGPD_E_ARG, "chann must be 3 or 12");
+    if (!workspace || ((uintptr_t)workspace & 255)) return fail(PGPD_E_WORKSPACE, "workspace is null or not 256-byte aligned");
+    const int cap = proj::project_capacity(workspace_bytes, P, chann);
+    if (cap < 0) return fail(PGPD_E_WORKSPACE, "workspace too small (see pgpd_gpd_project_workspace_bytes)");
+    if (cap > 0 && !idx) return fail(PGPD_E_ARG, "idx is null");
+    proj::ProjWs w;
+    proj::plan_project(workspace, P, cap, chann, w);
+    proj::project(pc, P, frames, G, offsets, idx, cap, chann, out, valid, w, (cudaStream_t)stream);
+    return check_cuda("pgpd_gpd_project");
 }
 
 }  // extern "C"

@@ -7,8 +7,12 @@ signatures, same on-disk layout ($PointNetGPD_FOLDER tree, SURVEY.md 7.4), same 
 
 Written from the reference's behaviour, not its code: one class parameterised by (views, classes).  The gripper-box
 crop is `crop_points` below (numpy, runs in DataLoader workers like the reference); the batched GPU version of the
-same crop is `pointnetgpd_b200.prep.crop`.  The GPD image projection (`projection=True`, used only by the GPD baseline
-scripts) is outside this package's scope and raises.
+same crop is `pointnetgpd_b200.prep.crop`.
+
+`projection=True` (the GPD baseline scripts, main_1v_gpd.py / main_fullv_gpd.py) yields the reference's 60 x 60 images
+instead: `(image float64 [project_chann, 60, 60], label[, object name])` or `None` (dataset.py:88-198,270).  The items
+are built on the CPU by `pointnetgpd_b200.projection` (numpy + cKDTree; the workers are forked after the script has
+initialised CUDA); `pointnetgpd_b200.prep.project` computes the same images for many grasps of a cloud on the GPU.
 """
 import glob
 import os
@@ -16,6 +20,8 @@ import pickle
 
 import numpy as np
 import torch.utils.data
+
+from .. import projection as _projection
 
 __all__ = ["BaseGraspDataset", "PointGraspDataset", "PointGraspMultiClassDataset", "PointGraspOneViewDataset",
            "PointGraspOneViewMultiClassDataset"]
@@ -75,7 +81,9 @@ class BaseGraspDataset(torch.utils.data.Dataset):
 
     def collect_pc(self, grasp, pc, transform):
         if self.projection:
-            raise NotImplementedError("GPD image projection is outside the scope of pointnetgpd_b200")
+            center, rows, width = grasp_frame(grasp, transform)
+            self.in_ind, img = _projection.project_grasp(pc, center, rows, width, self.project_chann)
+            return None if img is None else img.transpose(2, 1, 0)            # [x, y, c] like project_pc
         self.in_ind, pts = crop_points(grasp, pc, transform)
         return None if len(self.in_ind) < self.min_point_limit else pts
 
@@ -125,8 +133,11 @@ class _GraspDataset(BaseGraspDataset):
         pts = self.collect_pc(grasp, pc, transform)
         if pts is None:
             return None
-        n = len(pts)
-        pts = pts[np.random.choice(n, size=self.grasp_points_num, replace=not (n > self.grasp_points_num))].T
+        if self.projection:
+            pts = pts.transpose((2, 1, 0))
+        else:
+            n = len(pts)
+            pts = pts[np.random.choice(n, size=self.grasp_points_num, replace=not (n > self.grasp_points_num))].T
         score = grasp[-2] + grasp[-1] * 0.01
         if self.MULTI_CLASS:
             label = 0 if score >= self.thresh_bad else (2 if score <= self.thresh_good else 1)

@@ -1,10 +1,10 @@
 """Host side of the data preparation in front of the model (SURVEY.md section 8f rows 1-2):
-gripper-box crop of a cloud for a batch of grasps, and resampling of every crop to exactly N points -- both run in
-libpgpd on the GPU; this module computes the per-grasp frames (a handful of 3x3 products per grasp) and drives the
-two-pass crop (count, prefix-sum, gather).
+gripper-box crop of a cloud for a batch of grasps, resampling of every crop to exactly N points, and the GPD
+baseline's 60 x 60 image projection of every crop -- all run in libpgpd on the GPU; this module computes the per-grasp
+frames (a handful of 3x3 products per grasp) and drives the two-pass crop (count, prefix-sum, gather).
 
 Reference semantics: BaseGraspDataset.collect_pc (PointNetGPD/model/dataset.py:15-76), the resampling of
-dataset.py:438-444 / dex-net/apps/kinect2grasp.py:473-478.
+dataset.py:438-444 / dex-net/apps/kinect2grasp.py:473-478, the projection of dataset.py:78-198.
 """
 import ctypes as C
 
@@ -82,3 +82,28 @@ def resample(pts, offsets, N, repeat=1, seed=0, return_index=False, lib=None):
     A.check(lib, lib.pgpd_resample(_ptr(src), _ptr(off_dev), C_, N, repeat, C.c_ulonglong(seed & (2**64 - 1)),
                                    _ptr(x), _ptr(oi), stream))
     return (x, oi) if return_index else x
+
+
+def project(pc, frames, chann, lib=None):
+    """GPD input images of one cloud for G grasps (BaseGraspDataset.collect_pc with projection=True, dataset.py:15-198).
+    pc: [P,3] float32 tensor (cuda); frames: [G,15] float64 (grasp_frames); chann: 3 or 12.  Returns (images
+    [G,chann,60,60] float32 on pc's device, the layout GPDClassifier reads; valid [G] bool: the box holds >= 50 points,
+    where the reference's item is None the image is all zeros).  Crop with pgpd_crop_box, then pgpd_gpd_project."""
+    if chann not in (3, 12):
+        raise ValueError("chann must be 3 or 12 (dataset.py:218-219)")
+    lib = lib or A.load()
+    dev = pc.device
+    pc = pc.contiguous().float()
+    offsets, _pts, idx = crop(pc, frames, lib=lib)
+    fr = torch.as_tensor(np.ascontiguousarray(frames), dtype=torch.float64, device=dev)
+    G, P, total = fr.shape[0], pc.shape[0], int(offsets[-1])
+    nbytes = lib.pgpd_gpd_project_workspace_bytes(P, G, total, chann)
+    ws = torch.empty(nbytes + 256, dtype=torch.uint8, device=dev)
+    out = torch.empty((G, chann, 60, 60), dtype=torch.float32, device=dev)
+    valid = torch.empty(G, dtype=torch.bool, device=dev)
+    stream = torch.cuda.current_stream(dev).cuda_stream if dev.type == "cuda" else None
+    idx = idx if total > 0 else torch.zeros(1, dtype=torch.int32, device=dev)
+    off_dev = offsets.to(dev)
+    A.check(lib, lib.pgpd_gpd_project(_ptr(pc), P, _ptr(fr), G, _ptr(off_dev), _ptr(idx), chann, _ptr(out), _ptr(valid),
+                                      (ws.data_ptr() + 255) & ~255, nbytes, stream))
+    return out, valid
